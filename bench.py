@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- tokens/s of single-batch decode through libcalm_b200.so (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--engine E]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one token of single-sequence decode (one pass of the per-token forward() path).  The
 N = 1 workload is BASELINE.json configs[1]: Llama-3-8B shape, random-init fp8 (e5m2) weights, 4096-token
@@ -253,6 +253,9 @@ def main():
     ap.add_argument("--kvbits", type=int, default=16, choices=[16, 8], help="KV cache element: fp16 (what the reference uses up to 4096 positions) or e5m2 (its choice beyond, run.c:537-539)")
     ap.add_argument("--layers", type=int, default=None, help="(debug) override the layer count")
     ap.add_argument("--pos0", type=int, default=None, help="(debug) first timed position instead of the end of the context")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write what they returned as DIR/<name>.npy: greedy_tokens (the device loop's tokens), "
+                         "greedy_last_logits (its last step's logits), e2e_last_logits (forward_cuda's logits of the host-stepped loop's last step)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
 
@@ -270,7 +273,6 @@ def main():
 
     import torch
 
-    from calm_b200 import build as cbuild
     from calm_b200 import lib
 
     rank, world, local = dist_setup(args.gpus)
@@ -289,8 +291,7 @@ def main():
     os.environ.setdefault("CALM_B200_QUIET", "1")  # keep stdout to the one JSON line
     sampler = ClockSampler(local)  # started well ahead of the timed region: nvidia-smi needs a second to come up on an 8-GPU box
     sampler.start()
-    cbuild.build()
-    L = lib.load()
+    L = lib.load()  # built by build(): the bench compiles nothing, its tree may be read-only
     seq_len = 4096
     tp = None
     if use_dist and args.parallel == "tp":
@@ -324,6 +325,7 @@ def main():
     barrier()
     t_wall1 = time.time()
     launches = int(L.calm_b200_launch_count() - l0)
+    dump = {"greedy_tokens": toks.astype(np.float64), "greedy_last_logits": dm.device_logits()} if args.dump_outputs else None
     ms = max_over_ranks(ms)
     value = K / (ms / 1e3) if is_tp else agg.whole_job_rate(K, ms)  # TP: the N GPUs serve ONE token stream
 
@@ -340,6 +342,11 @@ def main():
         tok = int(np.argmax(np.ctypeslib.as_array(p, shape=(spec.vocab_size,))))
     torch.cuda.synchronize()
     e2e_s = max_over_ranks(time.perf_counter() - t0)
+    if dump is not None and rank == 0:
+        dump["e2e_last_logits"] = np.ctypeslib.as_array(p, shape=(spec.vocab_size,)).copy()
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     clocks = sampler.stop(t_wall0, time.time())  # both timed regions (device loop, then host-stepped loop)
     barrier()
     e2e = K / e2e_s if is_tp else agg.whole_job_rate(K, e2e_s * 1e3)

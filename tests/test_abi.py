@@ -49,10 +49,7 @@ def test_no_oracle_in_product():
     assert "oracle" not in out and "calm_ref" not in out
 
 
-def test_struct_layout_matches_reference_header(tmp_path):
-    """include/calm_model.h vs reference src/model.h, field by field (only where the reference is mounted);
-    the ctypes mirror vs include/calm_model.h everywhere."""
-    prog = r'''
+LAYOUT_PROG = r'''
 #include <stdio.h>
 #include <stddef.h>
 #include HEADER
@@ -69,16 +66,24 @@ int main() {
   printf("MAX_LAYERS %d MAX_EXPERTS %d KV_SINKS %d FF %d\n", MAX_LAYERS, MAX_EXPERTS, KV_SINKS, FF_UPDATE_KV_ONLY);
   return 0; }
 '''
-    def layout(header):
-        src = tmp_path / "l.c"
-        src.write_text(prog.replace("HEADER", '"%s"' % header))
-        exe = tmp_path / "l"
-        subprocess.run(["/usr/bin/gcc", str(src), "-o", str(exe)], check=True)
-        return subprocess.run([str(exe)], capture_output=True, text=True, check=True).stdout
 
-    ours = layout(os.path.join(ROOT, "include", "calm_model.h"))
-    if os.path.exists("/root/reference/src/model.h"):
-        assert ours == layout("/root/reference/src/model.h")
+
+def struct_layout(header, workdir):
+    """Sizes and field offsets of the model records declared by `header`, as printed by LAYOUT_PROG."""
+    src = os.path.join(workdir, "l.c")
+    with open(src, "w") as f:
+        f.write(LAYOUT_PROG.replace("HEADER", '"%s"' % header))
+    exe = os.path.join(workdir, "l")
+    subprocess.run(["/usr/bin/gcc", src, "-o", exe], check=True)
+    return subprocess.run([exe], capture_output=True, text=True, check=True).stdout
+
+
+def test_struct_layout_matches_reference_header(tmp_path):
+    """include/calm_model.h vs reference src/model.h, field by field (tests/golden/reference-layout.txt is the same
+    program's output over the reference header, tools/make_golden.py); the ctypes mirror vs include/calm_model.h."""
+    ours = struct_layout(os.path.join(ROOT, "include", "calm_model.h"), str(tmp_path))
+    with open(os.path.join(ROOT, "tests", "golden", "reference-layout.txt")) as f:
+        assert ours == f.read()
     kv = dict(line.rsplit(" ", 1) for line in ours.strip().splitlines()[:-1])
     for name, cls in (("Config", cstructs.Config), ("Weights", cstructs.Weights), ("RunState", cstructs.RunState), ("Transformer", cstructs.Transformer)):
         assert int(kv[name]) == C.sizeof(cls)

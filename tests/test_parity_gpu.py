@@ -2,7 +2,7 @@
 backend (upload_cuda -> prepare_cuda -> forward_cuda per token), against
   (1) the CPU oracle (oracle/calm_oracle.c) on the same seeded model,
   (2) the committed golden fixtures produced by the unmodified reference, and
-  (3) the unmodified reference itself (oracle/_ref/libcalm_ref_cpu.so) when it travelled to this box.
+  (3) stored teacher-forced runs of the unmodified reference at other seeds and positions.
 Tolerance (stated, DESIGN.md): |dlogit| <= 5e-3 * std(logits); argmax identical on every step whose
 reference top-2 margin exceeds twice that; KV entries within fp16 rounding."""
 import os
@@ -20,7 +20,7 @@ from calm_b200 import modelgen as mg  # noqa: E402
 from calm_b200.cstructs import FF_UPDATE_KV_ONLY  # noqa: E402
 
 sys.path.insert(0, os.path.join(ROOT, "tools"))
-from make_golden import GOLDEN_SPECS, model_digest  # noqa: E402
+from make_golden import GOLDEN_SPECS, load_ref_run, model_digest  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 
@@ -61,18 +61,16 @@ def test_logits_match_golden_and_oracle(oracle_pkg, name):
     ck.release(host)
 
 
-def test_against_live_reference(oracle_pkg):
-    """The unmodified reference CPU backend, executed on this box, different seed / positions."""
-    if not oracle_pkg.available("reference"):
-        pytest.skip("oracle/_ref/libcalm_ref_cpu.so did not travel")
+def test_against_live_reference():
+    """The unmodified reference CPU backend on a different seed / positions (golden reference-runs.npz: each step's
+    largest logits and a fixed random sample of the others)."""
     for name in ("tiny-llama", "tiny-moe", "tiny-gf4"):
         spec = mg.SPECS[name]
         toks = mg.teacher_tokens(spec.vocab_size, 20, start=50)
-        host = mg.HostModel(spec, seed=5)
-        ref = oracle_pkg.teacher_forced(oracle_pkg.Checker("reference"), host, toks)
+        idx, ref, sigma = load_ref_run(name, 5, 20, start=50)
         got = run_device(spec, 5, toks)
-        tol = TOL_SIGMA * ref.std()
-        assert np.abs(got - ref).max() <= tol, name
+        tol = TOL_SIGMA * sigma
+        assert np.abs(np.take_along_axis(got, idx, 1) - ref).max() <= tol, name
 
 
 def test_kv_only_flag_and_prompt_pipeline(oracle_pkg):
