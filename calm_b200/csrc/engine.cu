@@ -65,8 +65,9 @@ struct Engine {
 	size_t smem_up_ring = 0, smem_wo_ring = 0, smem_down_ring = 0;
 	bool attn2_cluster = false; // ... with the CTAs of a unit as one thread-block cluster (slices folded through distributed shared memory)
 	bool attn2 = false; // k_attn2 (attn.cuh): KV slice requested into shared memory ahead of the dependency wait
+	bool attn_mma = false; // k_attn_mma (attn.cuh): the same, scores and values on mma.sync (head_dim 128, 4 query heads per kv head)
 	int attn_nbmax = 0;
-	size_t attn2_smem = 0;
+	size_t attn2_smem = 0, attn_mma_smem = 0;
 
 	// launch plan (grid sizes / dynamic shared memory), fixed at prepare time
 	int grid_qkv = 0, grid_wo = 0, grid_up = 0, grid_down = 0, grid_out = 0;
@@ -443,6 +444,19 @@ void launch_attn2(const AttnArgs& a, int nunits, int* nl) {
 	++*nl;
 }
 
+template <typename KVT>
+void launch_attn_mma(const AttnArgs& a, int nunits, int* nl) {
+	if (!nl) { // prepare time: opt-in, and the cell fold's co-residency requirement (as k_attn2)
+		smem_optin(k_attn_mma<KVT>, g.attn_mma_smem);
+		int per_sm = 0;
+		CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_attn_mma<KVT>, ATTN_THREADS, g.attn_mma_smem));
+		if (per_sm * g.sms < nunits * a.nsplit) g.attn_mma = false;
+		return;
+	}
+	launch_pdl(k_attn_mma<KVT>, nunits * a.nsplit, ATTN_THREADS, g.attn_mma_smem, a);
+	++*nl;
+}
+
 // shapes k_attn2 is instantiated for: head_dim 128 with 4 or 8 query heads per kv head, head_dim 64 with 2, 4 or 8
 bool attn2_shape_ok(int hg, int lpp, int head_dim) {
 	return head_dim == lpp * 8 && ((lpp == 16 && (hg == 4 || hg == 8)) || (lpp == 8 && (hg == 2 || hg == 4 || hg == 8)));
@@ -450,6 +464,10 @@ bool attn2_shape_ok(int hg, int lpp, int head_dim) {
 
 template <typename KVT>
 void dispatch_attn(const AttnArgs& a, int nunits, int* nl) {
+	if (g.attn_mma) {
+		launch_attn_mma<KVT>(a, nunits, nl);
+		if (nl) return; // (at prepare time k_attn2 is set up as well: the co-residency check may have turned k_attn_mma off)
+	}
 	if (g.attn2) {
 		switch (g.attn_lpp * 100 + g.attn_hg) {
 		case 1604: launch_attn2<KVT, 4, 16>(a, nunits, nl); return;
@@ -745,6 +763,10 @@ void make_plan() {
 		const bool want = !(getenv("CALM_B200_ATTN2") && atoi(getenv("CALM_B200_ATTN2")) == 0);
 		g.attn2 = want && attn2_shape_ok(g.attn_hg, g.attn_lpp, c.head_dim) && g.attn_nbmax <= ATTN2_MAXB && g.attn2_smem <= 200 * 1024;
 		g.attn2_cluster = g.attn2 && g.attn_nsplit <= ATTN2_MAX_CLUSTER && getenv("CALM_B200_ATTN_CLUSTER") && atoi(getenv("CALM_B200_ATTN_CLUSTER")) != 0;
+		// k_attn_mma where it applies (CALM_B200_ATTN_MMA=0: k_attn2, for A/B runs in one build)
+		g.attn_mma_smem = attn_mma_smem_bytes<KVT>(g.attn_nbmax);
+		const bool want_mma = !(getenv("CALM_B200_ATTN_MMA") && atoi(getenv("CALM_B200_ATTN_MMA")) == 0);
+		g.attn_mma = want_mma && g.attn2 && !g.attn2_cluster && g.attn_hg == ATTN_MMA_HG && c.head_dim == ATTN_MMA_HD && g.attn_mma_smem <= 200 * 1024;
 		AttnArgs aa = {};
 		aa.head_dim = c.head_dim, aa.nsplit = g.attn_nsplit;
 		dispatch_attn<KVT>(aa, c.n_kv_heads * g.attn_qgroups, nullptr);
